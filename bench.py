@@ -2,6 +2,7 @@
 """Benchmark of the embed+detect hot path (BASELINE.json metric: embed+detect frames/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--card C] [--batch B] [--size S]
+                    [--dump-outputs DIR]
 
 One "step" = model.embed(batch, msgs, is_video=False) followed by model.detect(imgs_w, is_video=False) on one batch of
 synthetic frames (configs[1] of BASELINE.json by default: videoseal_1.0, 256-bit, 64 x 3x256x256 per GPU).  Under torchrun
@@ -12,6 +13,7 @@ all-gather of the [B, 1+K] logits that reassembles the detection output).  Print
 modules) on the host cores; the unmodified reference itself needs packages that are not installed here (DESIGN.md).
 """
 import argparse
+import atexit
 import json
 import os
 import re
@@ -44,7 +46,13 @@ def parse_args():
     ap.add_argument("--clip-frames", type=int, default=512)
     ap.add_argument("--no-hbm-leg", action="store_true", help="skip the 768x768 leg that measures the HBM-bound kernels")
     ap.add_argument("--profile-out", default="", help="write the per-kernel table (JSON) here")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what embed() and detect() returned in the last timed step as DIR/<name>.npy "
+                         "(float32; a seeded sample of the frames when they exceed 64 MB), to compare builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 class ClockSampler:
@@ -59,6 +67,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "50",
                                           "-i", str(self.idx)], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self.proc.kill)     # the sampler never outlives bench.py, also when it fails before stop()
             threading.Thread(target=self._read, daemon=True).start()
         except Exception:
             self.proc = None
@@ -156,6 +165,29 @@ def load_peaks():
         return {"hbm_gbs": d["hbm_gbs"], "tf_burst": d["bf16_tflops"], "tf_sustained": d.get("bf16_tflops_sustained", d["bf16_tflops"]),
                 "src": "measured"}
     return {"hbm_gbs": 6650.0, "tf_burst": 1590.0, "tf_sustained": 1400.0, "src": "fallback"}
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(outs: dict, out_dir: str, seed: int = 0):
+    """Write the per-frame outputs `outs` (name -> tensor with frames along dim 0) as out_dir/<name>.npy in float32.  When they
+    exceed DUMP_BYTES, the same seeded sample of frames (in frame order) is taken from every array."""
+    import numpy as np
+    import torch
+    n = next(iter(outs.values())).shape[0]
+    per_frame = sum(4 * t[0].numel() for t in outs.values())
+    keep = min(n, DUMP_BYTES // per_frame)
+    if keep == 0:
+        raise SystemExit(f"--dump-outputs: one frame of outputs is {per_frame} bytes, more than the {DUMP_BYTES}-byte budget")
+    idx = None
+    if keep < n:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:keep].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outs.items():
+        t = t.detach().float().cpu()
+        np.save(os.path.join(out_dir, name + ".npy"), (t if idx is None else t[idx]).numpy())
+    return {"dir": out_dir, "arrays": sorted(outs), "frames": n if idx is None else idx.tolist()}
 
 
 def build_card_on_disk(card_name: str, seed: int = 0):
@@ -404,13 +436,13 @@ def run_ours(args):
 
     def step_local(i):
         out = model.embed(imgs[i % NB], msgs_v if vid else msgs, is_video=vid)
-        return model.detect(out["imgs_w"], is_video=vid)["preds"]
+        return {**out, **model.detect(out["imgs_w"], is_video=vid)}
 
     def step(i):
-        preds = step_local(i)
+        outs = step_local(i)
         if world > 1:
-            dist.all_gather(gathered, preds)   # reassemble the detection output on every rank ([B,1+K] per rank)
-        return preds
+            dist.all_gather(gathered, outs["preds"])   # reassemble the detection output on every rank ([B,1+K] per rank)
+        return outs
 
     def sync_all():
         torch.cuda.synchronize()
@@ -429,8 +461,9 @@ def run_ours(args):
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     sync_all()
     ev0.record()
-    for i in range(args.steps):
+    for i in range(args.steps - 1):
         step(i)
+    last = step(args.steps - 1)
     ev1.record()
     sync_all()
     ms = ev0.elapsed_time(ev1)
@@ -441,6 +474,8 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = t.item()
     fps = world * B * args.steps / (ms / 1000.0)
+    dumped = dump_outputs(last, args.dump_outputs) if args.dump_outputs and rank == 0 else None
+    del last
 
     # ---- end-to-end through the C ABI with HOST buffers (pinned): H2D + embed + D2H, H2D + detect + D2H, every step
     e2e = None
@@ -619,6 +654,7 @@ def run_ours(args):
                        "l2": f"{NB} rotating input batches ({NB * B * 3 * S * S * 4 / 1e6:.0f} MB > 126 MB L2); activations per step >> L2"},
             "step_tflops": (fe * n_keys + fd * B) * world * args.steps / (ms / 1000.0) / 1e12,
             "clocks": clocks, "e2e": e2e, "gpu_launches": launches, "roofline": roofline, "roofline_hbm": roofline_hbm, "clip": clip, "cpu_baseline": cpu,
+            "dumped_outputs": dumped,
             "top_kernels": [{k: (round(v, 4) if isinstance(v, float) else v) for k, v in r.items()} for r in table[:8]],
         }
         sys.stdout.flush()

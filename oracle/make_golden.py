@@ -7,7 +7,9 @@
    (`load_state_dict(strict=False)` exactly like utils/cfg.py:148-149),
 3. checks oracle/restate.py against the reference outputs on seeded inputs (pins the oracle),
 4. writes small fixtures to tests/golden/<card>.pt: full logits, strided samples + global
-   statistics of the image-sized outputs, so the fixtures stay small.
+   statistics of the image-sized outputs, so the fixtures stay small.  The samples of the
+   six video-mode runs (case D) go to tests/golden/<card>_video_modes.pt so that no
+   fixture file exceeds 1 MB.
 """
 import math
 import os
@@ -206,6 +208,10 @@ def main(cards=None):
             out["cases"]["structured"] = {"H": 352, "W": 416, "msg_seed": 6, "imgs_w_s": sample(r["imgs_w"], 4), "hmaps_s": sample(hm, 4),
                                           "preds": d["preds"].clone(), "hmaps_stats": stats(hm), "oracle_vs_ref": errs}
         path = os.path.join(ROOT, "tests", "golden", card_name + ".pt")
+        if "vid_modes" in out["cases"]:
+            modes_path = os.path.join(ROOT, "tests", "golden", card_name + "_video_modes.pt")
+            torch.save({"card": card_name, "seed": SEED, "modes": out["cases"]["vid_modes"].pop("modes")}, modes_path)
+            print(card_name, "->", modes_path, os.path.getsize(modes_path) // 1024, "KiB")
         torch.save(out, path)
         print(card_name, "->", path, os.path.getsize(path) // 1024, "KiB", f"{time.time()-t0:.1f}s")
 

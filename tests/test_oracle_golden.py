@@ -82,12 +82,14 @@ def test_oracle_video_modes_lowres_and_aggregations_match_reference_golden(card)
     spec = restate.spec_from_card(load_card(card))
     orc = restate.OracleModel(spec, restate.synth_state_dict(spec, seed=gold["seed"]))
     c = gold["cases"]["vid_modes"]
+    modes = torch.load(os.path.join(ROOT, "tests", "golden", f"{card}_video_modes.pt"))
+    assert modes["seed"] == gold["seed"] and len(modes["modes"]) == 6
     g = torch.Generator().manual_seed(c["gen_seed"])
     vid = torch.rand(c["F"], 3, c["H"], c["W"], generator=g)
     msgs = torch.randint(0, 2, (1, spec["nbits"]), generator=g)
     orc.chunk_size, orc.step_size = c["chunk_size"], c["step_size"]
     with torch.no_grad():
-        for key, ref in c["modes"].items():
+        for key, ref in modes["modes"].items():
             mode, lowres = key.split("/")
             orc.video_mode = mode
             o = orc.embed(vid, msgs, is_video=True, lowres_attenuation=bool(int(lowres)))
